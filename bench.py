@@ -61,7 +61,25 @@ def parse():
     ap.add_argument("--momentum", type=float, default=0.0)
     ap.add_argument("--optimizer", default="auto", choices=["auto", "sgd", "adamw"],
                     help="auto: SGD lr=0.01 for CNNs (the reference benchmark), AdamW for BERT")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the device-timed steps, write what the last of them computed on rank 0 to "
+                         "DIR/<name>.npy (float32): its loss and a fixed sample of the updated parameters")
     return ap.parse_args()
+
+
+def dump_outputs(out_dir, torch, loss, model, max_params=1 << 22):
+    """loss.npy: the step's loss.  params.npy: the parameters after the step's update, flattened and concatenated in
+    model.parameters() order; above ``max_params`` values, the values at a fixed, seeded set of positions (sorted),
+    which keeps the files under 64 MB for any model."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().reshape(1).cpu().numpy())
+    flat = torch.cat([p.detach().float().reshape(-1) for p in model.parameters()])
+    if flat.numel() > max_params:
+        idx = torch.randint(0, flat.numel(), (max_params,), generator=torch.Generator().manual_seed(0)).unique()
+        flat = flat[idx.to(flat.device)]
+    np.save(os.path.join(out_dir, "params.npy"), flat.cpu().numpy())
 
 
 class ClockSampler:
@@ -154,6 +172,7 @@ def build(args, torch, bps, device):
     from byteps_b200.models import get_model
 
     is_bert = args.model.startswith("bert")
+    torch.manual_seed(1234)     # same initial weights on every run, so that two builds compute the same steps
     model = get_model(args.model)
     dt = torch.bfloat16 if args.dtype == "bf16" else torch.float32
     model = model.to(device)
@@ -326,8 +345,15 @@ def main():
     if bps.rank() == 0:
         sampler.start()
     # ---- device-timed region: inputs resident on the device (the reference's benchmark does the same)
-    ms = timed(lambda i: stepper(), args.steps)
+    last_loss = [None]
+
+    def timed_step(i):
+        last_loss[0] = stepper()
+    ms = timed(timed_step, args.steps)
     note("device-timed region done: %.3f ms/step" % (ms / args.steps))
+    if args.dump_outputs and bps.rank() == 0:
+        dump_outputs(args.dump_outputs, torch, last_loss[0], model)
+        note("outputs written to %s" % args.dump_outputs)
     if use_graph:
         # kernels of ours inside one captured step (graph replays do not pass through python launch counters)
         gs = getattr(opt, "grad_sync", None)

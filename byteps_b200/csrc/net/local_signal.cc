@@ -19,6 +19,10 @@ LocalComm::LocalComm(int local_rank, const std::vector<int>& members, const std:
       suffix_(suffix) {
   BPS_CHECK(!members_.empty());
   root_ = *std::max_element(members_.begin(), members_.end());
+  // sun_path holds 107 bytes: a longer path would be cut short, and two ranks could end up on the same socket
+  for (int r : members_) {
+    BPS_CHECK_LT(path_of(r).size(), sizeof(sockaddr_un::sun_path)) << "socket path too long: " << path_of(r);
+  }
   fd_ = socket(AF_UNIX, SOCK_DGRAM, 0);
   BPS_CHECK_GE(fd_, 0) << "socket() failed";
   std::string p = path_of(rank_);

@@ -1,5 +1,6 @@
 import os
 import sys
+import tempfile
 
 import pytest
 
@@ -27,3 +28,20 @@ def pytest_collection_modifyitems(config, items):
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
         if "multigpu" in item.keywords and ngpu < 2:
             item.add_marker(pytest.mark.skip(reason="needs >= 2 GPUs"))
+
+
+@pytest.fixture(autouse=True)
+def _no_gpu_for_cpu_tests(request, monkeypatch):
+    """A test without the gpu mark checks the CPU path: the processes it starts see no GPU, as on a machine without
+    one.  (On a one-GPU machine its ranks would otherwise all take cuda:0, and NCCL refuses ranks that share a
+    device.)"""
+    if request.node.get_closest_marker("gpu") is None:
+        monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
+
+
+@pytest.fixture
+def sock_dir():
+    """A short directory for Unix-domain sockets: a socket path holds at most 107 bytes, which tmp_path under a
+    long TMPDIR can exceed."""
+    with tempfile.TemporaryDirectory(prefix="bps", dir="/tmp") as d:
+        yield d

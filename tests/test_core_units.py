@@ -838,14 +838,14 @@ def _host_reduce_rank(rank, world, tag, tmp):
         assert hr.signals_received() == 3 * 9 * (world - 1)       # READY, shard done and BCAST_READY per follower per round
 
 
-def test_host_local_reduce_three_ranks(tmp_path):
+def test_host_local_reduce_three_ranks(sock_dir):
     """csrc/core/host_reduce.h by itself: slots in shared memory, READY / DO_BROADCAST / BCAST_READY datagrams,
     CpuReducer sum on the root, window reuse across rounds."""
     import os
 
     from _mp import run_workers
 
-    run_workers(_host_reduce_rank, world=3, args=("unit%d" % os.getpid(), str(tmp_path)), timeout=120)
+    run_workers(_host_reduce_rank, world=3, args=("unit%d" % os.getpid(), sock_dir), timeout=120)
 
 
 def _host_reduce_timeouts(rank, world, tag, tmp):
@@ -877,9 +877,9 @@ def _host_reduce_timeouts(rank, world, tag, tmp):
     assert np.all(out == world)
 
 
-def test_host_local_reduce_timeouts_do_not_hang(tmp_path):
+def test_host_local_reduce_timeouts_do_not_hang(sock_dir):
     import os
 
     from _mp import run_workers
 
-    run_workers(_host_reduce_timeouts, world=2, args=("tmo%d" % os.getpid(), str(tmp_path)), timeout=120)
+    run_workers(_host_reduce_timeouts, world=2, args=("tmo%d" % os.getpid(), sock_dir), timeout=120)

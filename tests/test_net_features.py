@@ -140,13 +140,13 @@ def test_colocated_ipc_moves_payload_through_shm():
     cl.stop()
 
 
-def test_uds_local_signalling(tmp_path):
+def test_uds_local_signalling(sock_dir):
     c = _core()
     members = [0, 1, 2]
     comms = {}
 
     def make(r):
-        comms[r] = c.LocalComm(r, members, str(tmp_path), "t")
+        comms[r] = c.LocalComm(r, members, sock_dir, "t")
     ts = [threading.Thread(target=make, args=(r,)) for r in members]
     for t in ts:
         t.start()
@@ -168,6 +168,12 @@ def test_uds_local_signalling(tmp_path):
         assert comms[r].recv_from_root(2000) == (2, c.SIG_DO_GROUP, 0)
     assert comms[0].recv_from_root(300) is None
     comms.clear()
+
+
+def test_uds_path_too_long_is_an_error():
+    c = _core()
+    with pytest.raises(RuntimeError, match="socket path too long"):
+        c.LocalComm(0, [0, 1], "/tmp/" + "d" * 120, "t")
 
 
 def test_multi_lane_connections_stripe_keys():

@@ -215,4 +215,5 @@ PYBIND11_MODULE(_cuda, m) {
   bind_cuda_ext(m);
   bind_cuda_ring(m);
   bind_cuda_compress(m);
+  bind_cuda_clip(m);
 }

@@ -6,3 +6,4 @@
 void bind_cuda_ext(pybind11::module_& m);
 void bind_cuda_ring(pybind11::module_& m);
 void bind_cuda_compress(pybind11::module_& m);
+void bind_cuda_clip(pybind11::module_& m);

@@ -89,6 +89,21 @@ def resync_fused_masters():
             s.sync_master_from_params()
 
 
+def clip_update_grid(numels: List[int], itemsize: int, world: int) -> int:
+    """CTAs of the clipped update (phase 3) over buckets of `numels` padded elements.  The kernel ends in a barrier
+    that pairs the CTAs of equal index across ranks, so the grid must be the same on every rank: it is sized from
+    rank 0's shard, the largest (shard_units), not from this rank's, which can be smaller or empty.  Nothing overlaps
+    phase 3 (it runs after backward), so it may take two CTAs per SM of a B200 (148 SMs); a fixed cap rather than the
+    local device's SM count keeps the grid rank-independent."""
+    tiles = 0
+    for n in numels:
+        groups = n // 8
+        per = (groups + world - 1) // world                   # rank 0's shard, in groups of 8 elements
+        units = per * 8 * itemsize // 16                      # 16-byte wire units
+        tiles += (units + 255) // 256                          # 256 units per tile (kClipTileUnits)
+    return max(1, min(tiles, 2 * 148))
+
+
 _HP_FMT = "<9f3if3i"   # matches csrc/kernels/pushpull.cuh::OptHParams (64 bytes)
 
 
@@ -97,10 +112,16 @@ class BucketedGradSync:
 
     def __init__(self, engine, param_groups, *, fused: Optional[str] = None, wire_dtype: Optional[torch.dtype] = None,
                  bucket_bytes: Optional[int] = None, backward_passes_per_step: int = 1, average: bool = True,
-                 priority_of: Optional[Dict] = None):
+                 priority_of: Optional[Dict] = None, max_grad_norm: Optional[float] = None):
         self.engine = engine
         self.world, self.rank = engine.size, engine.rank
         self.fused = fused                     # None | "sgd" | "adam" | "adamw"
+        # global-norm clipping inside the fused exchange (pushpull_clip.cu): phase 1 per bucket from the hooks,
+        # norm (phase 2) and clipped update + parameter all-gather (phase 3) from synchronize()
+        self.clip = max_grad_norm is not None
+        self.max_grad_norm = max_grad_norm
+        if self.clip and not fused:
+            raise ValueError("max_grad_norm inside the exchange needs a fused optimizer")
         self.average = average
         self.bpps = backward_passes_per_step
         self.bucket_bytes = bucket_bytes or _env_int("BYTEPS_BUCKET_BYTES", 16 << 20)
@@ -109,6 +130,10 @@ class BucketedGradSync:
         params = [(gi, p) for gi, g in enumerate(param_groups) for p in g["params"] if p.requires_grad]
         if not params:
             raise ValueError("no parameters require gradients")
+        if (self.clip and wire_dtype in (torch.bfloat16, torch.float16)
+                and any(p.dtype == torch.float32 for _, p in params)):
+            raise ValueError("max_grad_norm cannot be combined with a wire cast of fp32 gradients "
+                             "(Compression.fp16/bf16): the clipped exchange keeps gradients in the parameter dtype")
         self.device = params[0][1].device
         for _, p in params:
             if p.device != self.device or not p.is_cuda:
@@ -129,7 +154,7 @@ class BucketedGradSync:
             cur.params.append(p)
             cur.starts.append(cur.numel)
             cur.numel += _pad8(p.numel())
-        # ---- arena layout: [grad windows][param windows (fused)][staging (wire cast)]
+        # ---- arena layout: [grad windows][param windows (fused)][staging (wire cast)][clip norm publish]
         off = 0
         for b in self.buckets:
             b.grad_off = off
@@ -143,6 +168,9 @@ class BucketedGradSync:
         if self._needs_stage():
             self.stage_bytes = max(self._wire_bytes(b) for b in self.buckets)
             off += (self.stage_bytes + 255) // 256 * 256
+        self.clip_pub_off = off
+        if self.clip:
+            off += 256
         cfg = engine.cfg
         stamp("buckets: layout of %d buckets, arena %d MiB" % (len(self.buckets), off >> 20))
         self.ctx = SymmContext(engine.group, self.device, max(off, 4096), cfg.symm_mode, cfg.use_nvls)
@@ -246,9 +274,39 @@ class BucketedGradSync:
             b.state0 = torch.zeros(n, dtype=torch.float32, device=self.device)
             b.state1 = torch.zeros(n, dtype=torch.float32, device=self.device) if kind != "sgd" else None
         ng = len(self.param_groups)
-        self._hp_dev = torch.zeros((ng, 64), dtype=torch.uint8, device=self.device)
+        # clip mode: one more row holds the ClipState {max_norm, norm, coef, step}, so refresh_hparams writes
+        # max_norm together with the groups in one launch
+        self._hp_dev = torch.zeros((ng + int(self.clip), 64), dtype=torch.uint8, device=self.device)
         self._group_step = [0] * ng
         self.loss_scale = 1.0
+        if self.clip:
+            self._init_clip()
+
+    def _init_clip(self):
+        cu = self.ctx.cu
+        ng = len(self.param_groups)
+        self._clip_state_ptr = self._hp_dev.data_ptr() + 64 * ng
+        self._grad_norm = self._hp_dev[ng, 4:8].view(torch.float32)[0]
+        # phase-1 partial sums, [bucket][CTA]; entries of CTAs a bucket does not launch stay zero
+        self._clip_slots = torch.zeros(len(self.buckets) * cu.CLIP_SLOTS_PER_BUCKET, dtype=torch.float64,
+                                       device=self.device)
+        # phase 3: one static table of ClipDesc per dtype, built once (graph-safe)
+        kind = cu.OPT_SGD if self.fused == "sgd" else cu.OPT_ADAM
+        nstreams = 2 if kind == cu.OPT_SGD else 3
+        by_dtype: Dict[torch.dtype, List[Bucket]] = {}
+        for b in self.buckets:
+            by_dtype.setdefault(b.dtype, []).append(b)
+        self._clip_tables = []
+        for dtype, bs in by_dtype.items():
+            rows = [[b.grad_off, b.param_off, b.numel, b.master.data_ptr(), b.state0.data_ptr(),
+                     b.state1.data_ptr() if b.state1 is not None else 0, self._hp_dev.data_ptr() + 64 * b.group_index,
+                     0] for b in bs]
+            table = torch.tensor(rows, dtype=torch.int64, device=self.device)
+            assert table.element_size() * table.shape[1] == cu.CLIP_DESC_BYTES
+            per_stage = nstreams * 256 * (16 // dtype.itemsize) * 4
+            stages = max(2, min(8, (96 << 10) // per_stage))
+            blocks = clip_update_grid([b.numel for b in bs], dtype.itemsize, self.world)
+            self._clip_tables.append((wire_code(dtype), kind, table, len(bs), blocks, stages))
 
     def sync_master_from_params(self):
         for b in self.buckets:
@@ -297,6 +355,8 @@ class BucketedGradSync:
                         float(g.get("eps", 1e-8)), 1.0 - b1 ** t, 1.0 - b2 ** t, 0,
                         int(self.fused == "adamw"), int(t == 1), 1.0 / self.loss_scale, 0, 0, 0)
             blob += struct.pack(_HP_FMT, *vals)
+        if self.clip:
+            blob += struct.pack("<f", float(self.max_grad_norm))    # ClipState.max_norm, right behind the groups
         self.ctx.cu.write_blob(self._hp_dev.data_ptr(), blob, cur.cuda_stream)
         self.engine.launches += 1
 
@@ -390,6 +450,13 @@ class BucketedGradSync:
         if self.fused:
             kind = cu.OPT_SGD if self.fused == "sgd" else cu.OPT_ADAM
             hp_ptr = self._hp_dev.data_ptr() + 64 * b.group_index
+            if self.clip:
+                # phase 1 only: the update waits for the global norm (_clip_tail)
+                slots = self._clip_slots.data_ptr() + 8 * cu.CLIP_SLOTS_PER_BUCKET * b.index
+                cu.clip_reduce_sumsq(view, wire_code(wire), b.grad_off, b.numel, scale, slots, hp_ptr, blocks,
+                                     self.threads, 0, nvls, cs.cuda_stream)
+                self._after_launch(b, cur, cs, ev_t)
+                return
             if wire == b.dtype and self._fused_engine == "tma":
                 # optimizer state streamed through shared memory with bulk copies (pushpull.cu, TMA variant)
                 es = 4 if b.dtype == torch.float32 else 2
@@ -471,7 +538,9 @@ class BucketedGradSync:
         self._ring_credit = credit * self.engine.cfg.partition_bound() if credit > 0 else 0
         self._stamps = os.environ.get("BYTEPS_COMM_STAMPS", "1") not in ("0", "")
         self._stamp_base = None
-        eligible = (self._reduce_engine in ("auto", "nvls", "lsu") and len(self.buckets) <= cu.RING_SLOTS
+        # clip mode has no ring variant: phase 1 goes out per bucket
+        eligible = (not self.clip and self._reduce_engine in ("auto", "nvls", "lsu")
+                    and len(self.buckets) <= cu.RING_SLOTS
                     and not (self.fused and self._fused_engine == "tma" and self.world == 1 and mode == "auto"))
         if mode == "auto":
             # one rank: nothing to wait for, the TMA-streamed optimizer kernel per bucket is the fastest;
@@ -657,6 +726,7 @@ class BucketedGradSync:
                 b.pending = 0
                 self._issue(b)
         self._ring_flush()
+        self._clip_tail()
         if self._stamps and self._last_done is not None:
             self.ctx.cu.ring_stamp(self.ctx.view, 1, self.comm_stream.cuda_stream)   # last exchange finished
             self._count_launch()
@@ -684,10 +754,37 @@ class BucketedGradSync:
                 b.pending = 0
                 self._issue(b)
         self._ring_flush()
+        self._clip_tail()
         if self._stamps and self._last_done is not None:
             self.ctx.cu.ring_stamp(self.ctx.view, 1, self.comm_stream.cuda_stream)   # last exchange finished
             self._count_launch()
         self._reset(keep_events=True)
+
+    def _clip_tail(self):
+        """Clip mode, after every bucket's phase 1: the global norm (phase 2), then the clipped update and parameter
+        all-gather (phase 3) on the comm stream.  The comm stream first waits for the current stream, so the new
+        parameters cannot land under a kernel of this step that still reads the old ones."""
+        if not self.clip:
+            return
+        cu, view, cs = self.ctx.cu, self.ctx.view, self.comm_stream
+        cs.wait_stream(torch.cuda.current_stream(self.device))
+        cu.clip_finalize(view, self._clip_slots.data_ptr(), self._clip_slots.numel(), self.clip_pub_off,
+                         self._clip_state_ptr, 0, cs.cuda_stream)
+        nvls = bool(self.ctx.nvls)
+        for wire, kind, table, n, blocks, stages in self._clip_tables:
+            cu.clip_update(view, wire, kind, table.data_ptr(), n, self._clip_state_ptr, blocks, stages, nvls, 0,
+                           cs.cuda_stream)
+        self._count_launch(1 + len(self._clip_tables))
+        done = torch.cuda.Event()
+        done.record(cs)
+        for b in self.buckets:        # the parameters of every bucket change only now
+            b.done = done
+        self._last_done = done
+
+    def grad_norm(self) -> torch.Tensor:
+        """Clip mode: 0-dim fp32 device tensor with the total gradient norm of the last step (before clipping).
+        Always the same storage, so CUDA-graph replays update it."""
+        return self._grad_norm
 
     def _flush_trace(self):
         """Turn the timing events of this step into Chrome-trace spans (device time, anchored at

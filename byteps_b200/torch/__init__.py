@@ -17,6 +17,7 @@ parameters instead of the gradients.
 from __future__ import annotations
 
 import io
+import math
 import os
 from contextlib import contextmanager
 
@@ -61,9 +62,18 @@ def _fused_kind(optimizer_cls, param_groups):
     return None
 
 
+def _check_max_grad_norm(v):
+    if v is None:
+        return None
+    v = float(v)
+    if not math.isfinite(v) or v <= 0:
+        raise ValueError("max_grad_norm must be a finite number > 0, got %r" % v)
+    return v
+
+
 class _DistributedOptimizer(torch.optim.Optimizer):
     def __init__(self, params, named_parameters, compression, backward_passes_per_step=1, fused_update=None,
-                 bucket_bytes=None, compression_params=None):
+                 bucket_bytes=None, compression_params=None, max_grad_norm=None):
         super(self.__class__, self).__init__(params)
         self._compression = compression
         from ..common.compression_params import translate
@@ -72,6 +82,11 @@ class _DistributedOptimizer(torch.optim.Optimizer):
         named_parameters = list(named_parameters) if named_parameters is not None else []
         self._enable_async = (int(os.getenv('BYTEPS_ENABLE_ASYNC', 0)) != 0)
         self._async_seeded = False
+        self._max_grad_norm = _check_max_grad_norm(max_grad_norm)
+        self._grad_norm = None
+        if self._enable_async and self._max_grad_norm is not None:
+            raise ValueError("max_grad_norm is not supported with BYTEPS_ENABLE_ASYNC=1: workers push weight deltas, "
+                             "there is no averaged gradient to clip")
         if self._enable_async:
             assert int(os.getenv('DMLC_NUM_WORKER', 1)) > 1, "Async is only valid for distributed training"
         if any(not isinstance(p, tuple) for p in named_parameters):
@@ -126,7 +141,8 @@ class _DistributedOptimizer(torch.optim.Optimizer):
             self._sync = BucketedGradSync(eng, self.param_groups, fused=kind, wire_dtype=_wire_of(compression),
                                           bucket_bytes=bucket_bytes,
                                           backward_passes_per_step=backward_passes_per_step,
-                                          priority_of=self._priority)
+                                          priority_of=self._priority,
+                                          max_grad_norm=self._max_grad_norm if kind else None)
             if kind:
                 self._sync.refresh_hparams()
         elif size() > 1 or eng.backend == "ps":
@@ -267,7 +283,32 @@ class _DistributedOptimizer(torch.optim.Optimizer):
             set_learning_rate(self.param_groups[0]["lr"])     # error feedback rescales by lr_prev/lr
         if self._should_sync:
             self.synchronize()
+        if self._max_grad_norm is not None:
+            params = [p for g in self.param_groups for p in g["params"] if p.requires_grad]
+            self._grad_norm = torch.nn.utils.clip_grad_norm_(params, self._max_grad_norm)
         return super(self.__class__, self).step(closure)
+
+    @property
+    def max_grad_norm(self):
+        return self._max_grad_norm
+
+    @max_grad_norm.setter
+    def max_grad_norm(self, value):
+        if value is None or self._max_grad_norm is None:
+            raise ValueError("max_grad_norm can be changed, not switched on or off, after construction")
+        self._max_grad_norm = _check_max_grad_norm(value)
+        if self._fused:
+            self._sync.max_grad_norm = self._max_grad_norm
+            self._sync.refresh_hparams()      # eager: reaches the next step; graphs: refresh_hparams() before replay
+
+    def grad_norm(self):
+        """With ``max_grad_norm``: the total L2 norm of the averaged gradients of the last step, before clipping (what
+        ``clip_grad_norm_`` returns), as a 0-dim fp32 tensor.  On the fused path it is one device tensor that every
+        step (and CUDA-graph replay) overwrites; reading it does not synchronise.  ``None`` without clipping, or
+        before the first step on the other paths."""
+        if self._fused and self._sync.clip:
+            return self._sync.grad_norm()
+        return self._grad_norm
 
     @property
     def grad_sync(self):
@@ -275,7 +316,8 @@ class _DistributedOptimizer(torch.optim.Optimizer):
 
 
 def DistributedOptimizer(optimizer, named_parameters=None, compression=Compression.none,
-                         backward_passes_per_step=1, fused_update=None, bucket_bytes=None, compression_params=None):
+                         backward_passes_per_step=1, fused_update=None, bucket_bytes=None, compression_params=None,
+                         max_grad_norm=None):
     """Wrap ``optimizer`` so gradients are averaged over all processes before
     ``step()``; communication overlaps with ``loss.backward()``.
 
@@ -287,12 +329,30 @@ def DistributedOptimizer(optimizer, named_parameters=None, compression=Compressi
     turns on lossy gradient compression per tensor - GPU kernels over NVLink, or the
     worker/server compressors in CPU-server mode.
 
-    ``synchronize()`` forces completion (e.g. before gradient clipping),
-    ``skip_synchronize()`` lets a following ``step()`` skip it.
+    ``max_grad_norm`` (a finite float > 0) clips the averaged gradients of every
+    ``step()`` to that global L2 norm before the update, with the semantics of
+    ``torch.nn.utils.clip_grad_norm_`` over every parameter that requires grad (one
+    without a gradient counts as zero; the norm is of the gradients after the loss
+    scale is removed; a NaN/inf norm propagates like in torch).  ``grad_norm()``
+    returns the norm before clipping; ``opt.max_grad_norm`` may be changed between
+    steps (under ``GraphedStep`` it reaches the kernels through ``refresh_hparams``,
+    like ``lr``).  With ``fused_update=True`` the norm is computed on the device
+    between the reduction and the update, inside the exchange, with no host
+    synchronisation.  After such a step this rank's shard of each bucket in ``p.grad``
+    holds the averaged gradient, the rest this rank's local one; as without clipping,
+    the gradient buffers are otherwise unspecified after ``step()``.  On every other
+    path ``step()`` calls ``clip_grad_norm_`` between ``synchronize()`` and the
+    wrapped optimizer's step.  Not available with ``BYTEPS_ENABLE_ASYNC=1`` or with
+    ``Compression.fp16/bf16`` on fp32 parameters of the fused path.
+
+    ``synchronize()`` forces completion (e.g. before gradient clipping without
+    ``max_grad_norm``; on the fused path it has already applied the update, so clip
+    with ``max_grad_norm`` there), ``skip_synchronize()`` lets a following
+    ``step()`` skip it.
     """
     cls = type(optimizer.__class__.__name__, (optimizer.__class__,), dict(_DistributedOptimizer.__dict__))
     return cls(optimizer.param_groups, named_parameters, compression, backward_passes_per_step, fused_update,
-               bucket_bytes, compression_params)
+               bucket_bytes, compression_params, max_grad_norm)
 
 
 def broadcast_parameters(params, root_rank, prefix="Parameter."):

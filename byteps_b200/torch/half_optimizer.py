@@ -13,7 +13,7 @@ from __future__ import annotations
 
 import torch
 
-from . import DistributedOptimizer
+from . import DistributedOptimizer, _check_max_grad_norm
 
 
 class HalfPrecisionDistributedOptimizer:
@@ -25,7 +25,7 @@ class HalfPrecisionDistributedOptimizer:
     scale halves on overflow (step skipped) and doubles after ``scale_window`` clean steps."""
 
     def __init__(self, optimizer, named_parameters=None, loss_scale: float = 1.0, dynamic_loss_scale: bool = False,
-                 scale_window: int = 1000, bucket_bytes=None):
+                 scale_window: int = 1000, bucket_bytes=None, max_grad_norm=None):
         self.loss_scale = float(loss_scale)
         self.dynamic = bool(dynamic_loss_scale)
         self.scale_window = int(scale_window)
@@ -33,6 +33,9 @@ class HalfPrecisionDistributedOptimizer:
         self.skipped_steps = 0
         self._masters = None
         if self.dynamic:
+            # the fp32 master gradients are clipped after unscaling, in _dynamic_step
+            self._max_grad_norm = _check_max_grad_norm(max_grad_norm)
+            self._grad_norm = None
             named = list(named_parameters) if named_parameters is not None else None
             self._opt = DistributedOptimizer(optimizer, named_parameters=named, fused_update=False,
                                              bucket_bytes=bucket_bytes)
@@ -49,8 +52,9 @@ class HalfPrecisionDistributedOptimizer:
                 g["params"] = masters
             self._sync = self._opt.grad_sync
             return
+        # static scale: the clipped norm is of the unscaled gradients because the kernels fold 1/loss_scale into it
         self._opt = DistributedOptimizer(optimizer, named_parameters=named_parameters, fused_update=True,
-                                         bucket_bytes=bucket_bytes)
+                                         bucket_bytes=bucket_bytes, max_grad_norm=max_grad_norm)
         self._sync = self._opt.grad_sync
         if self._sync is not None:
             self._sync.loss_scale = self.loss_scale
@@ -92,6 +96,9 @@ class HalfPrecisionDistributedOptimizer:
         for p in halves:
             m = self._masters[p]
             m.grad = p.grad.detach().float().mul_(inv)
+        if self._max_grad_norm is not None:
+            masters = [m for g in self._opt.param_groups for m in g["params"] if m.requires_grad]
+            self._grad_norm = torch.nn.utils.clip_grad_norm_(masters, self._max_grad_norm)
         # the wrapped optimizer's own update (on the masters), bypassing the distributed step's second sync
         type(self._opt).__mro__[1].step(self._opt)
         with torch.no_grad():
@@ -109,6 +116,25 @@ class HalfPrecisionDistributedOptimizer:
             self._sync.loss_scale = self.loss_scale
             self._sync.refresh_hparams()
         return self._opt.step(closure)
+
+    @property
+    def max_grad_norm(self):
+        return self._max_grad_norm if self._masters is not None else self._opt.max_grad_norm
+
+    @max_grad_norm.setter
+    def max_grad_norm(self, value):
+        if self._masters is None:
+            self._opt.max_grad_norm = value       # static scale: the fused exchange reads it
+            return
+        if value is None or self._max_grad_norm is None:
+            raise ValueError("max_grad_norm can be changed, not switched on or off, after construction")
+        self._max_grad_norm = _check_max_grad_norm(value)
+
+    def grad_norm(self):
+        """Total norm of the last step's unscaled, averaged gradients before clipping (``max_grad_norm``)."""
+        if self._masters is not None:
+            return self._grad_norm
+        return self._opt.grad_norm()
 
     def master_params(self):
         if self._masters is not None:

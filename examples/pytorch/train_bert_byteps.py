@@ -20,6 +20,8 @@ p.add_argument("--seq-len", type=int, default=128)
 p.add_argument("--steps", type=int, default=20)
 p.add_argument("--warmup-steps", type=int, default=5)
 p.add_argument("--no-cuda", action="store_true", help="CPU run over gloo (unfused optimizer, fp32)")
+p.add_argument("--max-grad-norm", type=float, default=None,
+               help="clip the averaged gradients to this global L2 norm every step (default: no clipping)")
 args = p.parse_args()
 bps.init()
 cuda = torch.cuda.is_available() and not args.no_cuda
@@ -30,7 +32,8 @@ model = get_model(args.model).to(dev)
 if cuda:
     model = model.to(torch.bfloat16)
 opt = bps.DistributedOptimizer(torch.optim.AdamW(model.parameters(), lr=1e-4, weight_decay=0.01),
-                               named_parameters=model.named_parameters(), fused_update=cuda)
+                               named_parameters=model.named_parameters(), fused_update=cuda,
+                               max_grad_norm=args.max_grad_norm)
 bps.broadcast_parameters(model.state_dict(), root_rank=0)
 ids = torch.randint(0, 30522, (args.batch_size, args.seq_len), device=dev)
 labels = torch.randint(0, 30522, (args.batch_size, args.seq_len), device=dev)
